@@ -2,6 +2,7 @@
 """bench.py -- the POMS hot path on B200: MG-preconditioned CG to 1e-10 relative residual.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c5|c2|c3|c4|c1] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is ONE complete MG-PCG solve (b = 1 on every DOF, x0 = 0) of the synthetic
 -Lap(u)+u problem of the chosen BASELINE config; `value` = DOF / (seconds per solve), inputs
@@ -14,17 +15,25 @@ axis 1, 512 element planes per GPU (weak scaling).
 --impl reference times the reference's CPU algorithm (oracle port: the reference itself is
 pure Python over an absent third-party package and cannot travel) on the host cores, on a
 bounded sample of the same workload.
+
+--dump-outputs DIR writes what the last timed solve returned (see dump_outputs) so that two builds
+can be compared output for output; the inputs are the same on every run with the same arguments.
+The bench writes nothing into the source tree, which may be read-only.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 CONFIGS = {
     # name: (ndim, p, elements per axis, description)
@@ -108,6 +117,16 @@ def pin_cpu_threads():
     return n
 
 
+def numba_cache_outside_tree():
+    """The CPU port compiles with numba cache=True, which writes next to its source (or fails at
+    import when no cache location is writable): point numba at a temporary directory instead, unless
+    the caller chose one.  Must run before numba is imported."""
+    if "NUMBA_CACHE_DIR" not in os.environ:
+        d = tempfile.mkdtemp(prefix="poms_b200_numba_")
+        atexit.register(shutil.rmtree, d, True)
+        os.environ["NUMBA_CACHE_DIR"] = d
+
+
 def cpu_port_solve(ndim, p, N, tol=1e-10, smoother="glt", Nc=8, ratio=4.0):
     """One MG-PCG solve with the CPU port of the same algorithm: oracle/poms_oracle_mt.py (numba,
     all host threads), or the single-threaded NumPy oracle if numba is unavailable.  b = A x0 like
@@ -151,6 +170,46 @@ def resolve_smoother(name, p):
 def cpu_sample_size(ndim):
     # bounded sample: ~10-30 s of CPU work
     return 128 if ndim == 3 else 1024
+
+
+DUMP_SAMPLE = 1 << 22       # entries of x written by --dump-outputs: 32 MB of float64
+
+
+def dump_indices(npts):
+    """Flat row-major indices into the global grid of the x entries --dump-outputs writes: every
+    point when there are at most DUMP_SAMPLE, else a sorted sample drawn with a fixed seed (C5:
+    515^3 points, 1.1 GB in full)."""
+    import numpy as np
+    n = int(np.prod(npts))
+    if n <= DUMP_SAMPLE:
+        return np.arange(n)
+    return np.unique(np.random.default_rng(0).integers(0, n, DUMP_SAMPLE))
+
+
+def dump_outputs(path, x, info, world, rank):
+    """Write what mg_pcg returned to the caller as path/<name>.npy, all float64: x.npy (x at
+    dump_indices(V.npts), gathered over the slabs), residual_history.npy, and the scalars niter,
+    restarts, success, res_norm, res_norm0.  Collective when world > 1; rank 0 writes."""
+    import numpy as np
+    import torch
+    V = x.space
+    dev = x.data.device
+    sub = np.unravel_index(dump_indices(V.npts), V.npts)
+    own = (sub[0] >= V.starts[0]) & (sub[0] <= V.ends[0])
+    loc = tuple(torch.as_tensor(s[own] - (V.starts[0] if a == 0 else 0), device=dev)
+                for a, s in enumerate(sub))
+    xs = torch.zeros(len(own), dtype=torch.float64, device=dev)
+    xs[torch.as_tensor(np.flatnonzero(own), device=dev)] = x.data[loc]
+    if world > 1:
+        torch.distributed.all_reduce(xs)        # every sampled point is owned by exactly one slab
+    if rank != 0:
+        return
+    out = {"x": xs.cpu().numpy(), "residual_history": np.asarray(info["history"], dtype=np.float64)}
+    for k in ("niter", "restarts", "success", "res_norm", "res_norm0"):
+        out[k] = np.float64(info[k])
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 _JSON_OUT = None
@@ -245,7 +304,13 @@ def main():
                     help="where the 1-D setup of the hierarchy runs (device: csrc/poms_setup.cu)")
     ap.add_argument("--no-exact-glt", action="store_true",
                     help="skip the extra solves with the reference's exact GLT smoother (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the solution and solver info of the last timed "
+                         "step to DIR/<name>.npy (float64; x sampled at fixed points, at most 34 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
+    numba_cache_outside_tree()
     pin_cpu_threads()
     _claim_stdout()
     rank = int(os.environ.get("RANK", "0"))
@@ -367,6 +432,9 @@ def main():
     launches = L.poms_launch_count() - l0
     ms = e0.elapsed_time(e1) / args.steps
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # now: x is the hierarchy's persistent solution vector, which the passes below overwrite
+        dump_outputs(args.dump_outputs, x, info, world, rank)
     # ---- separate instrumented pass (CUDA events around every kernel family) for the roofline and
     # the per-kernel breakdown: its event records perturb the latency-bound coarse levels, so it
     # is kept out of the headline timing above
