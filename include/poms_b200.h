@@ -320,6 +320,36 @@ int poms_halo_exchange_p2p(const double* src_lo, double* dst_lo, const double* s
                            int64_t n_doubles, void* my_flags, void* lo_flags, void* hi_flags,
                            void* stream);
 
+/*
+ * Finite-element quadrature on tensor-product B-spline spaces (poms_fem3d.cu; poms_b200/fem.py builds the
+ * tables).  Both entry points march along axis 1 over one chunk of element planes; a 2-D space is passed
+ * with a middle axis of one coefficient and one quadrature point.
+ *  poms_quad_to_coef_3d: y (+)= (B1^T (x) B2^T (x) B3^T) F, F = (e1_hi - e1_lo) * q1n quadrature planes of
+ *    shape (m2, m3) with pitches fld / fpld.  Axis 1: element e touches rows s1[e] .. s1[e]+k1n-1 with the
+ *    weighted values b1[(e * k1n + k) * q1n + q]; rows below `store_from` are added to y, the others
+ *    stored.  Axis 2: row r = sum_t c2[r * w2 + t] * (quadrature row st2[r] + t).  Axis 3: row r =
+ *    sum_{m, q} c3[r * (p+1)^2 + m (p+1) + q] * F[(e3[r] + m)(p+1) + q], ne3 elements.  The *_host
+ *    arrays are host copies of s1, st2, e3 (checks and tile sizes).  Deterministic, no atomics.
+ *  poms_quad_error_3d: out[0] (+)= sum w (ref[0] - u_h)^2, and with grad out[1] (+)= sum w |ref[1..3] -
+ *    grad u_h|^2 (a null gradient component is skipped) over quadrature planes j1_lo .. j1_lo+nq1-1 of
+ *    m1; ref[c] has row / plane pitches rld[c] / rpld[c] (host arrays of 4).  Per quadrature point j of
+ *    axis a: first coefficient s_a[j], k_a values v_a[j * k_a + i] and derivatives d_a, weight w_a[j];
+ *    k3 = p+1.  ws: the library workspace (deterministic grid reduction).
+ */
+int poms_quad_to_coef_3d(const double* F, int64_t fld, int64_t fpld, double* y, int64_t ld, int64_t pld,
+                         int n1, int n2, int n3, int m2, int m3, int p, int e1_lo, int e1_hi, int k1n,
+                         int q1n, const int32_t* s1, const double* b1, int store_from, const int32_t* st2,
+                         const double* c2, int w2, const int32_t* e3, const double* c3, int ne3,
+                         const int32_t* s1_host, const int32_t* st2_host, const int32_t* e3_host,
+                         void* stream);
+int poms_quad_error_3d(const double* x, int64_t ld, int64_t pld, int n1, int n2, int n3, int m2, int m3, int p,
+                       const double* const* ref, const int64_t* rld, const int64_t* rpld, int j1_lo, int nq1,
+                       int k1n, const int32_t* s1, const double* v1, const double* d1, const double* w1,
+                       int k2n, const int32_t* s2, const double* v2, const double* d2, const double* w2,
+                       const int32_t* s3, const double* v3, const double* d3, const double* w3,
+                       const int32_t* s1_host, const int32_t* s2_host, const int32_t* s3_host, int m1,
+                       int grad, int accumulate, double* out, void* ws, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

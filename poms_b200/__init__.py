@@ -12,6 +12,7 @@ Module names mirror the reference's `sources/` directory so that
                   KronSumMatrix
     mg            Transfer, CoarseSolver, two_grid; EXTENSION: Hierarchy, vcycle, mg_pcg
     dist          slab partition along axis 1, halo exchange, all-reduce (NCCL)
+    fem           EXTENSION: load_vector (b_i = int f phi_i), error_norms (L2 / H1), evaluate
 
 All arithmetic runs in hand-written CUDA kernels (csrc/poms_kernels.cu) behind the C ABI of
 include/poms_b200.h; there is no CPU fallback.

@@ -65,6 +65,11 @@ _PROTOS = {
     "poms_knot_insertion_rows": (C.c_int, [_vp, _i, _vp, _i, _i, _vp, _vp, _vp]),
     "poms_band_lu_nopiv": (C.c_int, [_vp, _i, _i, _vp, _vp, _vp]),
     "poms_axis_dense_dmma": (C.c_int, [_vp, _vp, _vp, _i, _i, _l, _l, _l, _l, _l, _l, _vp]),
+    "poms_quad_to_coef_3d": (C.c_int, [_vp, _l, _l, _vp, _l, _l, _i, _i, _i, _i, _i, _i, _i, _i, _i,
+                                      _i, _vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
+    "poms_quad_error_3d": (C.c_int, [_vp, _l, _l, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _i,
+                                    _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                    _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "poms_ipc_alloc": (C.c_int, [_l, C.POINTER(C.c_void_p)]),
     "poms_ipc_free": (C.c_int, [_vp]),
     "poms_ipc_handle_bytes": (C.c_int, []),

@@ -100,6 +100,21 @@ def assemble_1d_bands(p, T, toeplitz_interior=True):
     return M, K
 
 
+def quadrature_tables(T, p):
+    """Per-element Gauss-Legendre tables of the (p+1)-point rule of `assemble_1d_bands` on the non-empty
+    knot spans of T: points x (ne, p+1), weights w (ne, p+1), basis values v and first derivatives d
+    (ne, p+1 functions, p+1 points) and the index `first` (ne,) of each element's first basis function."""
+    T = np.asarray(T, dtype=float)
+    n = len(T) - p - 1
+    spans = np.array([k for k in range(p, n) if T[k + 1] > T[k]], dtype=np.int64)
+    a, b = T[spans], T[spans + 1]
+    u, w = np.polynomial.legendre.leggauss(p + 1)
+    x = 0.5 * (a + b)[:, None] + 0.5 * (b - a)[:, None] * u[None, :]
+    wq = 0.5 * (b - a)[:, None] * w[None, :]
+    v, dv = _all_basis(T, p, spans, x)
+    return {"n": n, "x": x, "w": wq, "v": v, "d": dv, "first": spans - p}
+
+
 def _is_uniform_open(T, p):
     """True if T is a clamped knot vector with equally spaced simple interior knots."""
     n = len(T) - p - 1
