@@ -718,6 +718,56 @@ def test_tma_matvec3d_emulated(tma_exes, tmp_path, san, p, N, variant):
         assert rel(y, x + dr) < tol and abs(dot - np.vdot(dr, dr)) < 1e-13 * dot
 
 
+@pytest.mark.parametrize("san", ["asan", "tsan"])
+@pytest.mark.parametrize("case", ["graded23", "graded1", "synthetic"])
+def test_tma_matvec3d_emulated_nonuniform(tma_exes, tmp_path, san, case):
+    """The operator on inputs the uniform cases never produce (tests/test_gpu_nonuniform.py runs them on
+    the GPU).  graded23: power-graded axes 2 and 3 leave one asymmetric Toeplitz row, so the host code
+    sends a variant-1 request to the round-1 kernel (variant 0), whose whole-tile fix-up then runs on
+    every other column and row.  graded1: a graded axis 1 keeps variant 1 but leaves it no steady plane
+    range.  synthetic: uniform bands with Toeplitz ranges that start and end off the 2p margins and off
+    the tile edges (the column-pair and plane-range arithmetic of both variants)."""
+    import test_gpu_nonuniform as nu
+    _core(san, True, case == "graded23")
+    EPI, FORM = _consts()
+    # graded23: N = 70 keeps the asymmetry of the graded rows (9e-3) within two decades of the threshold
+    p, N = 3, {"graded23": (12, 70, 70), "graded1": (20, 20, 70), "synthetic": (20, 36, 140)}[case]
+    kinds = {"graded23": ("u", "pow", "pow"), "graded1": ("pow", "u", "u"), "synthetic": ("u", "u", "u")}[case]
+    knots = [nu.family_knots(k, p, n) for k, n in zip(kinds, N)]
+    MK = [bs.assemble_1d_bands(p, T) for T in knots]
+    ms, ks = [m for m, k in MK], [k for m, k in MK]
+    ks[2] = ks[2] + ms[2]
+    nf = [m.shape[0] for m in ms]
+    coef, rg = _toeplitz_tables(ms, ks, p)
+    for a in range(3):
+        assert nu.range_ok(kinds[a], p, nf[a], *rg[2 * a:2 * a + 2])
+    sym = all(np.all(np.abs(r - r[::-1]) <= 1e-13 * np.abs(r).max()) for a in (1, 2) for r in coef[a])
+    assert sym == (case != "graded23")
+    if case == "synthetic":
+        # hi1 - lo1 >= 2p: planes whose window ends at row hi1 exist; lo3 even: at odd p the column pair
+        # (lo3 - 1, lo3) straddles the range start
+        rg = np.array([7, 16, 9, 30, 42, 101], dtype=np.int32)
+        for a in range(3):
+            ms[a], ks[a] = nu.perturb_outside([ms[a], ks[a]], rg[2 * a], rg[2 * a + 1], seed=a)
+    rng = np.random.default_rng(5)
+    x, b = rng.standard_normal(nf), rng.standard_normal(nf)
+    ab = po.apply_band
+    yo = (ab(ks[0], ab(ms[1], ab(ms[2], x, 2), 1), 0) + ab(ms[0], ab(ks[1], ab(ms[2], x, 2), 1), 0)
+          + ab(ms[0], ab(ms[1], ab(ks[2], x, 2), 1), 0))
+    ys = {}
+    for variant in (1, 0):
+        run = lambda epi, bb, om: _run_tma(tma_exes[san], tmp_path, p, FORM["sum"], EPI[epi], ms, ks, x, bb, om,
+                                           variant, (coef, rg))
+        dot, ys[variant] = run("store", None, 1.0)
+        assert rel(ys[variant], yo) < 1e-14
+        assert abs(dot - np.vdot(x, yo)) < 1e-13 * np.vdot(np.abs(x), np.abs(yo))
+        assert rel(run("resid", b, 1.0)[1], b - yo) < 1e-14
+        if san == "tsan":
+            break
+    if case == "graded23" and san == "asan":
+        assert np.array_equal(ys[1], ys[0]), "a variant-1 request must run variant 0 on asymmetric rows"
+
+
 # ------------------------------------------------------------------------------------------------
 # the 2-D fast path (BASELINE configs C2 and C4): warp-autonomous TMA mat-vec (kron_matvec2d_tma_kernel,
 # translation unit 7: private 4-stage ring of 2-D boxes per warp, no CTA barrier in the march) through
