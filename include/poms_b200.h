@@ -350,6 +350,35 @@ int poms_quad_error_3d(const double* x, int64_t ld, int64_t pld, int n1, int n2,
                        const int32_t* s1_host, const int32_t* s2_host, const int32_t* s3_host, int m1,
                        int grad, int accumulate, double* out, void* ws, void* stream);
 
+/*
+ * Particle coupling on tensor-product B-spline spaces (poms_points.cu; poms_b200/fem.py: evaluate_points,
+ * deposit).  Axis a has n_a coefficients and the knot vector T_a (n_a + p + 1 entries, device memory); a
+ * 2-D space is passed with T2 = NULL and n2 = 1, and its points have d = 2 coordinates (axes 1 and 3).
+ * Points: pts[k * d + a], 0 <= m < 2^31, every coordinate inside [T_a[p], T_a[n_a]] (checked by the
+ * caller).  Span of x: T[k] <= x < T[k+1], x = T[n] in the last non-empty span.  Cell of a point: its
+ * span per axis, c_a = k_a - p, key = (c1 C2 + c2) C3 + c3 with C_a = n_a - p (C2 = 1 in 2-D).
+ *  poms_points_eval: u[k] = u_h(X_k) and, if g is not NULL, g[k * d + a] = d u_h / dx_a (X_k), for the
+ *    coefficients x[r1 * pld + r2 * ld + r3].
+ *  poms_points_locate: key[k] = the cell of point k.
+ *  poms_points_moments: for the cells of the cell planes c1_lo .. c1_hi-1 (cell l of the chunk: key
+ *    l + c1_lo C2 C3), mom[l * nt + (i1 k2n + i2)(p+1) + i3] = sum w_j phi1_i1 phi2_i2 phi3_i3 (X_j) over
+ *    the points j = perm[offs[l] .. offs[l+1]-1] of the cell, in that order; nt = (p+1)^2 k2n, k2n = p+1
+ *    (3-D) or 1 (2-D).
+ *  poms_points_assemble: rows r1 = c1_lo .. c1_hi-1+p of y receive the sum of the moments of their cells
+ *    in planes c1_lo .. c1_hi-1 (fixed order); rows r1 < store_from are added to, the others stored.
+ *    n2 = 1: 2-D.  Deterministic, no atomics.
+ */
+int poms_points_eval(const double* x, int64_t ld, int64_t pld, int n1, int n2, int n3, int p, const double* T1,
+                     const double* T2, const double* T3, const double* pts, int d, int64_t m, double* u,
+                     double* g, void* stream);
+int poms_points_locate(const double* pts, int d, int64_t m, int n1, int n2, int n3, int p, const double* T1,
+                       const double* T2, const double* T3, int64_t* key, void* stream);
+int poms_points_moments(const double* pts, const double* w, int d, const int64_t* perm, const int64_t* offs,
+                        int c1_lo, int c1_hi, int n1, int n2, int n3, int p, const double* T1,
+                        const double* T2, const double* T3, double* mom, void* stream);
+int poms_points_assemble(const double* mom, int c1_lo, int c1_hi, int n1, int n2, int n3, int p, double* y,
+                         int64_t ld, int64_t pld, int store_from, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

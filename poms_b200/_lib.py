@@ -70,6 +70,11 @@ _PROTOS = {
     "poms_quad_error_3d": (C.c_int, [_vp, _l, _l, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _i,
                                     _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                     _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
+    "poms_points_eval": (C.c_int, [_vp, _l, _l, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _l, _vp, _vp, _vp]),
+    "poms_points_locate": (C.c_int, [_vp, _i, _l, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "poms_points_moments": (C.c_int, [_vp, _vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp,
+                                      _vp]),
+    "poms_points_assemble": (C.c_int, [_vp, _i, _i, _i, _i, _i, _i, _vp, _l, _l, _i, _vp]),
     "poms_ipc_alloc": (C.c_int, [_l, C.POINTER(C.c_void_p)]),
     "poms_ipc_free": (C.c_int, [_vp]),
     "poms_ipc_handle_bytes": (C.c_int, []),

@@ -13,7 +13,8 @@ CSRC = os.path.join(HERE, "csrc")
 SRC = os.path.join(CSRC, "poms_kernels.cu")
 EXTRA_SRC = [os.path.join(CSRC, "poms_extra.cu"), os.path.join(CSRC, "poms_setup.cu"),
              os.path.join(CSRC, "poms_transfer3d_v2.cu"),
-             os.path.join(CSRC, "poms_fem3d.cu")]              # self-contained units (own kernels + C ABI)
+             os.path.join(CSRC, "poms_fem3d.cu"),
+             os.path.join(CSRC, "poms_points.cu")]             # self-contained units (own kernels + C ABI)
 OUT = os.path.join(HERE, "libpoms_b200.so")
 OBJDIR = os.path.join(ROOT, "build", "obj")
 TUS = [0, 1, 2, 3, 4, 5, 6, 7]

@@ -5,6 +5,9 @@ vectors).
     load_vector(V, knots, p, f)        b_i = int f phi_i dx              (kernel poms_quad_to_coef_3d)
     error_norms(x, knots, p, u, grad_u) ||u - u_h||_L2, |u - u_h|_H1     (kernel poms_quad_error_3d)
     evaluate(x, knots, p, points)      u_h on a tensor grid              (per-axis poms_axis_gather)
+    evaluate_points(x, knots, p, P)    u_h (and grad u_h) at points P    (kernel poms_points_eval)
+    deposit(V, knots, p, P, w)         b_i = sum_k w_k phi_i(P_k)        (poms_points_locate, a stable sort,
+                                                                          poms_points_moments / _assemble)
 
 Quadrature: the (p+1)-point Gauss-Legendre rule per element and axis of `bsplines.assemble_1d_bands`, so
 `load_vector` and the mass / stiffness bands of the solver integrate with the same points.
@@ -16,6 +19,11 @@ as broadcastable fp64 device tensors, (m1, 1, 1), (1, m2, 1), (1, 1, m3) in 3-D 
 `plane_chunk` element planes; by default as many as keep one array of chunk values within
 CHUNK_BYTES (1 GiB), so memory stays bounded at any grid size.  The contraction with the basis runs in
 the kernels; the values are read in place (any row and plane pitch, unit stride along the last axis).
+
+Particle coupling (evaluate_points, deposit): `points` is an (m, d) fp64 tensor on the space's device, each
+coordinate inside [T_a[p], T_a[n_a]].  A point belongs to the knot span T[k] <= x < T[k+1], a point at T[n]
+to the last non-empty span (scipy's BSpline and `evaluate` do the same), so on a breakpoint a derivative is
+the right-hand one.
 
 Slab-partitioned spaces are not supported yet (NotImplementedError).
 """
@@ -29,7 +37,7 @@ from . import bsplines as bs
 from .mg import _AxisOp, _pitch
 from .stencil import DeviceContext, StencilVector, _stream
 
-__all__ = ["load_vector", "error_norms", "evaluate", "CHUNK_BYTES"]
+__all__ = ["load_vector", "error_norms", "evaluate", "evaluate_points", "deposit", "CHUNK_BYTES"]
 
 CHUNK_BYTES = 1 << 30
 
@@ -269,3 +277,112 @@ def evaluate(x, knots, p, points):
         src, shape = dst, out_shape
     return src[..., :shape[-1]]
 
+
+def _points(knots, p, d, dev, points, weights=None):
+    """Check the points (and weights) of `evaluate_points` / `deposit` against a d-dimensional space whose
+    storage is on `dev`; returns (points, weights, knot tensor, per-axis knot pointers of the kernels' 3-D
+    view).  The range and finiteness check reads one flag from the device."""
+    if not isinstance(points, torch.Tensor) or points.dtype != torch.float64:
+        raise ValueError("points must be a float64 torch.Tensor")
+    if points.device != dev:
+        raise ValueError("points must be on %s (got %s)" % (dev, points.device))
+    if points.ndim != 2 or points.shape[1] != d:
+        raise ValueError("points must have shape (m, %d) (got %s)" % (d, tuple(points.shape)))
+    m = points.shape[0]
+    if m >= 1 << 31:
+        raise ValueError("at most 2^31 - 1 points per call (got %d)" % m)
+    if weights is not None:
+        if not isinstance(weights, torch.Tensor) or weights.dtype != torch.float64:
+            raise ValueError("weights must be a float64 torch.Tensor")
+        if weights.device != dev:
+            raise ValueError("weights must be on %s (got %s)" % (dev, weights.device))
+        if tuple(weights.shape) != (m,):
+            raise ValueError("weights must have shape (%d,) (got %s)" % (m, tuple(weights.shape)))
+        weights = weights.contiguous()
+    Ts = [np.asarray(T, dtype=float) for T in knots]
+    lo = torch.tensor([T[p] for T in Ts], dtype=torch.float64, device=dev)
+    hi = torch.tensor([T[len(T) - p - 1] for T in Ts], dtype=torch.float64, device=dev)
+    points = points.contiguous()
+    if m and not bool(((points >= lo) & (points <= hi)).all()):        # NaN and inf fail both comparisons
+        bad = ~((points >= lo) & (points <= hi))
+        k, a = (int(v) for v in bad.nonzero()[0])
+        raise ValueError("point %d has coordinate %r on axis %d; points must be finite and inside [%r, %r]"
+                         % (k, float(points[k, a]), a, float(lo[a]), float(hi[a])))
+    Tdev = torch.as_tensor(np.concatenate(Ts), dtype=torch.float64, device=dev)
+    offs = np.concatenate([[0], np.cumsum([len(T) for T in Ts])])
+    ptrs = [Tdev.data_ptr() + 8 * int(o) for o in offs[:-1]]
+    if d == 2:
+        ptrs = [ptrs[0], None, ptrs[1]]
+    return points, weights, Tdev, ptrs
+
+
+def evaluate_points(x, knots, p, points, grad=False):
+    """u_h = sum_i x_i phi_i at the rows of `points` ((m, d) fp64 on the device of x), as an (m,) tensor;
+    with grad=True, (u, g) with g[k] = grad u_h(points[k]), (m, d).  One thread per point: binary search
+    of each knot vector, the degree-p basis with first derivatives in registers, a gather of the (p+1)^d
+    coefficients.  Deterministic.  Raises ValueError for a wrong dtype, device or shape, a non-finite
+    coordinate or one outside [T_a[p], T_a[n_a]], and m >= 2^31; that check costs one device-to-host read."""
+    V = x.space
+    _check(V, knots, p)
+    d, dev = V.ndim, x._buf.device
+    points, _, Tdev, T = _points(knots, p, d, dev, points)
+    m = points.shape[0]
+    u = torch.empty(m, dtype=torch.float64, device=dev)
+    g = torch.empty((m, d), dtype=torch.float64, device=dev) if grad else None
+    if m:
+        n1, n2, n3, ld, pld = _geom(V)
+        _lib.check(_lib.lib().poms_points_eval(
+            x.flat.data_ptr(), ld, pld, n1, n2, n3, p, T[0], T[1], T[2], points.data_ptr(), d, m, u.data_ptr(),
+            g.data_ptr() if grad else None, _stream()), "poms_points_eval")
+    return (u, g) if grad else u
+
+
+def deposit(V, knots, p, points, weights, out=None, plane_chunk=None):
+    """b_i = sum_k weights[k] phi_i(points[k]) on the space V as a StencilVector (`out`: a vector of V whose
+    owned entries are all overwritten).  Point charges, a Monte-Carlo source or measurements as a
+    right-hand side; the adjoint of `evaluate_points`.
+
+    Deterministic (bit-identical on repeated calls) and free of atomics: a kernel gives every point its cell
+    (knot span per axis) as an int64 key, a stable torch.sort orders the points by cell, one warp per cell
+    sums the (p+1)^d basis products of its points in that order, and an output-centric kernel adds the
+    moments of the <= (p+1)^d cells of each coefficient in a fixed order.  Scratch: 16 B per point for the
+    sorted keys and the permutation (24 B while the sort runs), plus the moments of one chunk of
+    `plane_chunk` cell planes along axis 1, 8 (p+1)^d B per cell (default: as many planes as keep them
+    within CHUNK_BYTES).  Raises ValueError like `evaluate_points` (also for weights of the wrong dtype,
+    device or shape), with the same one device-to-host read."""
+    _check(V, knots, p)
+    if plane_chunk is not None and int(plane_chunk) < 1:
+        raise ValueError("plane_chunk must be >= 1")
+    if out is not None and not V.compatible(out.space):
+        raise ValueError("out is not a vector of V")
+    d = V.ndim
+    dev = out._buf.device if out is not None else torch.empty(0, device=V.device).device
+    points, weights, Tdev, T = _points(knots, p, d, dev, points, weights)
+    m = points.shape[0]
+    if out is None:
+        out = StencilVector(V, zero=False)
+    if m == 0:
+        out.data.zero_()
+        return out
+    n1, n2, n3, ld, pld = _geom(V)
+    C1, C2, C3 = n1 - p, (n2 - p if d == 3 else 1), n3 - p
+    nt = (p + 1) ** d
+    L = _lib.lib()
+    key = torch.empty(m, dtype=torch.int64, device=dev)
+    _lib.check(L.poms_points_locate(points.data_ptr(), d, m, n1, n2, n3, p, T[0], T[1], T[2], key.data_ptr(),
+                                    _stream()), "poms_points_locate")
+    skey, perm = torch.sort(key, stable=True)
+    del key
+    ch = int(plane_chunk) if plane_chunk is not None else max(1, CHUNK_BYTES // (8 * C2 * C3 * nt))
+    ch = min(ch, C1)
+    mom = torch.empty(ch * C2 * C3 * nt, dtype=torch.float64, device=dev)
+    for c0 in range(0, C1, ch):
+        c1 = min(C1, c0 + ch)
+        cells = torch.arange(c0 * C2 * C3, c1 * C2 * C3 + 1, dtype=torch.int64, device=dev)
+        offs = torch.searchsorted(skey, cells)
+        _lib.check(L.poms_points_moments(points.data_ptr(), weights.data_ptr(), d, perm.data_ptr(),
+                                         offs.data_ptr(), c0, c1, n1, n2, n3, p, T[0], T[1], T[2],
+                                         mom.data_ptr(), _stream()), "poms_points_moments")
+        _lib.check(L.poms_points_assemble(mom.data_ptr(), c0, c1, n1, n2, n3, p, out.flat.data_ptr(), ld, pld,
+                                          0 if c0 == 0 else c0 + p, _stream()), "poms_points_assemble")
+    return out
