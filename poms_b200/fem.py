@@ -3,6 +3,7 @@ tensor-product B-spline spaces of a `Hierarchy` (single device, 2-D and 3-D, p =
 vectors).
 
     load_vector(V, knots, p, f)        b_i = int f phi_i dx              (kernel poms_quad_to_coef_3d)
+    boundary_load(V, knots, p, g, a, s) b_i += int_F g phi_i ds on a face (kernel poms_quad_to_coef_3d)
     error_norms(x, knots, p, u, grad_u) ||u - u_h||_L2, |u - u_h|_H1     (kernel poms_quad_error_3d)
     evaluate(x, knots, p, points)      u_h on a tensor grid              (per-axis poms_axis_gather)
     evaluate_points(x, knots, p, P)    u_h (and grad u_h) at points P    (kernel poms_points_eval)
@@ -25,6 +26,10 @@ coordinate inside [T_a[p], T_a[n_a]].  A point belongs to the knot span T[k] <= 
 to the last non-empty span (scipy's BSpline and `evaluate` do the same), so on a breakpoint a derivative is
 the right-hand one.
 
+Boundary data (boundary_load): with `Hierarchy(..., c=c, robin=...)` the solver's operator is the weak form
+of -Lap u + c u = f with du/dn + alpha u = g on every face (alpha = 0: Neumann).  The right-hand side is
+`load_vector` for f plus one `boundary_load` per face where g is not zero.
+
 Slab-partitioned spaces are not supported yet (NotImplementedError).
 """
 import ctypes as C
@@ -37,7 +42,7 @@ from . import bsplines as bs
 from .mg import _AxisOp, _pitch
 from .stencil import DeviceContext, StencilVector, _stream
 
-__all__ = ["load_vector", "error_norms", "evaluate", "evaluate_points", "deposit", "CHUNK_BYTES"]
+__all__ = ["load_vector", "boundary_load", "error_norms", "evaluate", "evaluate_points", "deposit", "CHUNK_BYTES"]
 
 CHUNK_BYTES = 1 << 30
 
@@ -154,6 +159,9 @@ def _values(t, name, shape, device):
                          % (name, tuple(t.shape), tuple(shape))) from None
     t = t.expand(shape)                          # (broadcast dimensions: copied below)
     m3 = shape[-1]
+    if len(shape) == 1:
+        t = t.contiguous()
+        return t, m3, m3
     if len(shape) == 2:
         if t.stride(1) != 1 or t.stride(0) < m3:
             t = t.contiguous()
@@ -200,6 +208,83 @@ def load_vector(V, knots, p, f, out=None, plane_chunk=None):
             a2.row_coef.data_ptr(), a2.K * a2.Q, a3.row_e0_dev.data_ptr(), a3.row_coef.data_ptr(), a3.E,
             a1.first.ctypes.data, a2.row_q0.ctypes.data, a3.row_e0.ctypes.data, _stream()),
             "poms_quad_to_coef_3d")
+    return out
+
+
+def boundary_load(V, knots, p, g, axis, side, out=None, plane_chunk=None):
+    """b_i += int_F g phi_i ds on the face F = {x_axis = T_axis[p]} (side 0) or {x_axis = T_axis[n]}
+    (side 1): the boundary data of a Neumann condition du/dn = g or a Robin condition du/dn + alpha u = g
+    (with `Hierarchy(..., robin=...)`), for the weak form of -Lap u + c u = f.
+
+    `g` receives the quadrature coordinates of the d-1 face axes (increasing axis order, the fixed
+    coordinate omitted) like `load_vector`'s f: (m1, 1), (1, m2) on a 3-D face, one (m,) tensor on a 2-D
+    face.  On an open knot vector only the first (side 0) or last (side 1) basis function along `axis` is
+    non-zero on F, with value 1, so the result is a (d-1)-dimensional load vector in that coefficient
+    plane; every other entry is left alone.  `out=None`: a new zero vector with the face contribution
+    only; `out` given: added into it, so `load_vector` followed by one call per face with data gives the
+    whole right-hand side.  `plane_chunk`: element planes along the first face axis per evaluation of g
+    (3-D; a 2-D face is one piece).
+
+    The contraction runs in `poms_quad_to_coef_3d` with a singleton middle axis (the layout of a 2-D
+    load vector), rows added, never stored.  A face normal to one of the leading axes is written in
+    place: its coefficient plane has unit stride along the last axis.  A face normal to the last
+    (contiguous) axis has none, so it is contracted into a contiguous scratch plane (line in 2-D) and
+    added to the strided face plane: O(N^(d-1)) work and memory.  Deterministic."""
+    _check(V, knots, p)
+    d = V.ndim
+    if isinstance(axis, bool) or not isinstance(axis, (int, np.integer)) or not 0 <= axis < d:
+        raise ValueError("axis must be an integer in 0..%d (got %r)" % (d - 1, axis))
+    if isinstance(side, bool) or side not in (0, 1):
+        raise ValueError("side must be 0 (x = T[p]) or 1 (x = T[n]) (got %r)" % (side,))
+    T = np.asarray(knots[axis], dtype=float)
+    n = V.npts[axis]
+    end = T[:p + 1] if side == 0 else T[n:]
+    if np.any(end != end[0]):
+        raise ValueError("knot vector %d is not open at side %d: the face term needs p + 1 equal end knots"
+                         % (axis, side))
+    if plane_chunk is not None and int(plane_chunk) < 1:
+        raise ValueError("plane_chunk must be >= 1")
+    if out is None:
+        out = StencilVector(V)
+    elif not V.compatible(out.space):
+        raise ValueError("out is not a vector of V")
+    dev = out._buf.device
+    j = 0 if side == 0 else n - 1
+    face = [b for b in range(d) if b != axis]
+    single = _Axis.singleton(dev)
+    a3 = _Axis(np.asarray(knots[face[-1]], dtype=float), p, dev)
+    a1 = _Axis(np.asarray(knots[face[0]], dtype=float), p, dev) if d == 3 else single
+    ax = [a1, single, a3]
+    n1, n3 = a1.n, a3.n
+    if axis == d - 1:
+        # the face plane is strided along every axis: contract into a contiguous scratch plane
+        ld_s = _pitch(n3)
+        scratch = torch.zeros((n1, ld_s), dtype=torch.float64, device=dev)
+        y, ld, pld = scratch.data_ptr(), ld_s, ld_s
+    elif d == 2:                                                    # row j of the 2-D array
+        y, ld, pld = out.flat[j].data_ptr(), V.ld, V.ld
+    elif axis == 0:                                                 # plane j: rows along axis 1
+        y, ld, pld = out.flat[j].data_ptr(), V.ld, V.ld
+    else:                                                           # out[:, j, :]: rows along axis 0
+        y, ld, pld = out.flat[:, j].data_ptr(), V.ld, V.npts[1] * V.ld
+    m3 = a3.E * a3.Q
+    ch = _chunk(plane_chunk, ax, 1)
+    L = _lib.lib()
+    for E0 in range(0, a1.E, ch):
+        E1 = min(a1.E, E0 + ch)
+        if d == 2:
+            F, fld, fpld = _values(g(a3.coords), "g", (m3,), dev)
+        else:
+            xs = (a1.coords[E0 * a1.Q:E1 * a1.Q].view(-1, 1), a3.coords.view(1, -1))
+            F, fld, fpld = _values(g(*xs), "g", ((E1 - E0) * a1.Q, m3), dev)
+        _lib.check(L.poms_quad_to_coef_3d(
+            F.data_ptr(), fld, fpld, y, ld, pld, n1, 1, n3, 1, m3, p, E0, E1, a1.K, a1.Q,
+            a1.first_dev.data_ptr(), a1.b_elem.data_ptr(), n1, single.row_q0_dev.data_ptr(),
+            single.row_coef.data_ptr(), 1, a3.row_e0_dev.data_ptr(), a3.row_coef.data_ptr(), a3.E,
+            a1.first.ctypes.data, single.row_q0.ctypes.data, a3.row_e0.ctypes.data, _stream()),
+            "poms_quad_to_coef_3d")
+    if axis == d - 1:
+        out.flat[..., j].add_(scratch[:, :n3].reshape(out.flat[..., j].shape))
     return out
 
 

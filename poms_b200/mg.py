@@ -28,7 +28,7 @@ from . import bsplines as bs
 from . import profiling
 from .multilevels import knots_to_insert
 from .stencil import (StencilVectorSpace, StencilVector, KronSumMatrix, DeviceContext,
-                      _stream, EPI_STORE, EPI_RESID, EPI_DINV, EPI_AXPY)
+                      _stream, EPI_STORE, EPI_RESID, EPI_DINV, EPI_AXPY, reaction_robin)
 from .kron_product import BandLU, kron_solve_bnd, kron_solve_bnd_update
 from . import solvers
 
@@ -552,7 +552,10 @@ class Level:
 
 
 class Hierarchy:
-    """Dyadic hierarchy of nested spline spaces for -Lap u + u on [0,1]^d.
+    """Dyadic hierarchy of nested spline spaces for -Lap u + c u on [0,1]^d with du/dn + alpha u = 0
+    on the boundary (default c = 1, alpha = 0: the reference's problem; `KronSumMatrix.poisson`).
+    Every level has the same c and alpha: the prolongation keeps boundary values on open knot vectors,
+    so P^T A_f P = A_c holds with the reaction and Robin terms too.
 
     N: elements per axis on the fine level (int or per-axis sequence); every level halves each
     axis that still has more than `Nc` elements (coarsen='semi') or all axes together until one
@@ -560,15 +563,18 @@ class Hierarchy:
     """
 
     def __init__(self, p, N, ndim=None, Nc=8, device="cuda", smoother="glt", nu=1, ratio=4.0,
-                 safety=1.1, slab=None, lengths=None, min_planes=32, coarsen="semi", setup="host"):
+                 safety=1.1, slab=None, lengths=None, min_planes=32, coarsen="semi", setup="host",
+                 c=1.0, robin=None):
         """setup='device': the 1-D setup (assembly, knot-insertion rows, banded LU, eigenproblems)
-        runs on the GPU (setup_device.py); 'host' (default): NumPy / SciPy."""
+        runs on the GPU (setup_device.py); 'host' (default): NumPy / SciPy.
+        c, robin: reaction coefficient and Robin coefficients of every level's operator
+        (`KronSumMatrix.poisson`; ValueError for negative values or a singular operator)."""
         if setup == "device":
             from . import setup_device as sd
             with sd.device_setup(True, device):
                 self.__init__(p, N, ndim=ndim, Nc=Nc, device=device, smoother=smoother, nu=nu, ratio=ratio,
                               safety=safety, slab=slab, lengths=lengths, min_planes=min_planes,
-                              coarsen=coarsen, setup="host")
+                              coarsen=coarsen, setup="host", c=c, robin=robin)
             self.setup = "device"
             return
         self.setup = "host"
@@ -578,6 +584,7 @@ class Hierarchy:
         # along the slab axis (L_1 = number of GPUs) so that the elements stay cubes.
         self.lengths = [1.0] * len(N) if lengths is None else [float(v) for v in lengths]
         self.p, self.ndim = p, len(N)
+        self.c, self.robin = reaction_robin(c, robin, self.ndim)
         self.device = torch.device(device)
         self.smoother, self.nu, self.ratio, self.safety = smoother, nu, ratio, safety
         self.levels = []
@@ -600,7 +607,7 @@ class Hierarchy:
             lv = Level()
             lv.N = list(Ns)
             lv.knots = [bs.make_open_knots(p, n + p) * L for n, L in zip(Ns, self.lengths)]
-            lv.A = KronSumMatrix.poisson(p, lv.knots)
+            lv.A = KronSumMatrix.poisson(p, lv.knots, c=self.c, robin=self.robin)
             # a level stays slab-partitioned while every slab keeps at least `min_planes` planes
             # (and enough for the p-wide halo and the 2q interface planes of the partitioned solve);
             # below that the per-operation latency of the exchanges exceeds the work, so the level is
@@ -625,21 +632,13 @@ class Hierarchy:
             self._setup_smoother(lv)
 
     def _setup_smoother(self, lv):
-        p, d = self.p, self.ndim
+        p = self.p
         A = lv.A
         if self.smoother == "glt":
             q = max(2 * p - 1, 1)
             lv.glt_bands = [bs.glt_band(p, n, degree=q) for n in A.npts]
             lv.glt_lu = [BandLU.from_band(b, self.device) for b in lv.glt_bands]
-            # lambda_max(B^-1 A) ~ max_a mu(K_a) prod_{b != a} mu(M_b): 1-D generalised
-            # eigenvalues wrt T (accurate to ~1 % in 2-D/3-D, see DESIGN.md), times `safety`.
-            muM = [_gen_eig_max(A.mass_bands[a], lv.glt_bands[a]) for a in range(d)]
-            best = 0.0
-            for a in range(d):
-                Kb = A.Ks[a] + (A.mass_bands[a] if a != d - 1 else 0.0)  # K_a + M_a
-                muK = _gen_eig_max(bs.pad_band(Kb, A.P), bs.pad_band(lv.glt_bands[a], A.P))
-                best = max(best, muK * float(np.prod([muM[c] for c in range(d) if c != a])))
-            lv.lmax = self.safety * best
+            lv.lmax = self.safety * self._glt_lmax(lv)
         elif self.smoother == "glt_poly":
             # B^-1 ~ q(T) (x) .. (x) q(T): degree-3 Chebyshev approximation of the GLT solve, applied
             # as TWO fused Kronecker band passes (F1: half-bandwidth q, F2: 2q) instead of 2d
@@ -650,18 +649,25 @@ class Hierarchy:
             F = [bs.poly_inverse_factors(b_, 3) for b_ in lv.glt_bands]
             lv.S1 = KronSumMatrix([f[0] for f in F])
             lv.S2 = KronSumMatrix([f[1] for f in F])
-            muM = [_gen_eig_max(A.mass_bands[a], lv.glt_bands[a]) for a in range(d)]
-            best = 0.0
-            for a in range(d):
-                Kb = A.Ks[a] + (A.mass_bands[a] if a != d - 1 else 0.0)
-                muK = _gen_eig_max(bs.pad_band(Kb, A.P), bs.pad_band(lv.glt_bands[a], A.P))
-                best = max(best, muK * float(np.prod([muM[c] for c in range(d) if c != a])))
-            lv.lmax = self.safety * best    # q(t) t = 0.9 at the high-frequency end of the symbol
+            lv.lmax = self.safety * self._glt_lmax(lv)    # q(t) t = 0.9 at the high-frequency end of the symbol
         elif self.smoother == "jacobi":
             lv.lmax = self.safety * self._power_lmax_jacobi(lv)
         else:
             raise ValueError("smoother must be 'glt', 'glt_poly' or 'jacobi'")
         lv.lmin = lv.lmax / self.ratio
+
+    def _glt_lmax(self, lv):
+        """lambda_max(B^-1 A) ~ max_a mu(K_a + c M_a) prod_{b != a} mu(M_b), B = T (x) .. (x) T: 1-D
+        generalised eigenvalues wrt T (accurate to ~1 % in 2-D/3-D, see DESIGN.md).  K_a here is the
+        level's band, so it carries the Robin entries of its axis (and the last one c M already)."""
+        A, d = lv.A, self.ndim
+        muM = [_gen_eig_max(A.mass_bands[a], lv.glt_bands[a]) for a in range(d)]
+        best = 0.0
+        for a in range(d):
+            Kb = A.Ks[a] + (self.c * A.mass_bands[a] if a != d - 1 else 0.0)  # K_a + c M_a
+            muK = _gen_eig_max(bs.pad_band(Kb, A.P), bs.pad_band(lv.glt_bands[a], A.P))
+            best = max(best, muK * float(np.prod([muM[b] for b in range(d) if b != a])))
+        return best
 
     def _power_lmax_jacobi(self, lv, iters=30):
         """lambda_max(D^-1 A) by power iteration on the device (setup; deterministic start)."""

@@ -601,11 +601,39 @@ class StencilMatrix:
                    "poms_diag_scale")
 
 
+def reaction_robin(c, robin, ndim):
+    """Checked (c, robin) of `KronSumMatrix.poisson`: c as a float, robin as None or a list of ndim
+    (alpha_lo, alpha_hi) float pairs.  Raises ValueError for a negative or non-finite value, a wrong
+    number of pairs, and for c = 0 without a positive alpha (the operator would be singular: constants
+    are in its kernel)."""
+    try:
+        c = float(c)
+    except (TypeError, ValueError):
+        raise ValueError("c must be a number (got %r)" % (c,)) from None
+    if not np.isfinite(c) or c < 0.0:
+        raise ValueError("c must be finite and >= 0 (got %r)" % c)
+    if robin is not None:
+        try:
+            pairs = [tuple(float(v) for v in ab) for ab in robin]
+        except (TypeError, ValueError):
+            raise ValueError("robin must be None or %d pairs (alpha_lo, alpha_hi) of numbers" % ndim) from None
+        if len(pairs) != ndim or any(len(ab) != 2 for ab in pairs):
+            raise ValueError("robin must have one pair (alpha_lo, alpha_hi) per axis (%d)" % ndim)
+        for a, ab in enumerate(pairs):
+            if not all(np.isfinite(v) and v >= 0.0 for v in ab):
+                raise ValueError("robin coefficients must be finite and >= 0 (axis %d: %r)" % (a, ab))
+        robin = pairs
+    if c == 0.0 and (robin is None or not any(v > 0.0 for ab in robin for v in ab)):
+        raise ValueError("c = 0 needs a Robin coefficient alpha > 0 on at least one face: -Lap u with "
+                         "du/dn = 0 everywhere is singular (constants are in its kernel)")
+    return c, robin
+
+
 class KronSumMatrix:
     """Kronecker-structured operator on a d-dim tensor-product space (d = 2, 3).
 
     form == FORM_SUM:   A = sum_a  M_1 (x) .. K_a .. (x) M_d   (bands Ms[a], Ks[a]); the last
-                        K must already contain K+M for the reference weak form -Lap u + u.
+                        K must already contain K + c M for the weak form -Lap u + c u (`poisson`).
     form == FORM_SINGLE: A = A_1 (x) .. (x) A_d                 (bands Ms[a]).
     Narrower bands are zero-padded to the common half-bandwidth P = max(pads).
     """
@@ -635,16 +663,30 @@ class KronSumMatrix:
         self._dev = {}
 
     @classmethod
-    def poisson(cls, p, knots):
-        """-Lap(u)+u on the tensor-product space with the given per-axis knot vectors: the
-        operator `assembly_2d` builds (/root/reference/sources/matrix_assembler.py:82-179), as
-        K(x)M + M(x)(K+M) [2-D] / K(x)M(x)M + M(x)K(x)M + M(x)M(x)(K+M) [3-D]."""
+    def poisson(cls, p, knots, c=1.0, robin=None):
+        """-Lap(u) + c u with du/dn + alpha u = 0 on the boundary (the weak form's natural condition)
+        on the tensor-product space with the given per-axis knot vectors.  The defaults (c = 1, no
+        Robin term) are the operator `assembly_2d` builds (/root/reference/sources/matrix_assembler.py:
+        82-179), K(x)M + M(x)(K+M) [2-D] / K(x)M(x)M + M(x)K(x)M + M(x)M(x)(K+M) [3-D].
+
+        robin: None, or one pair (alpha_lo, alpha_hi) per axis: alpha int_F u v ds on the faces
+        x_a = T_a[p] and x_a = T_a[n_a].  On an open knot vector only the first (last) basis function
+        is non-zero there, with value 1, so the face term is (alpha e e^T) (x) M_others: one diagonal
+        entry of K_a.  c M(x)..(x)M goes into the last K as K + c M.  Both keep the Kronecker-sum
+        form and change no interior row.  c >= 0, alpha >= 0, and c > 0 or some alpha > 0 (otherwise
+        the operator is singular): ValueError."""
         from . import setup_device as sd
+        c, robin = reaction_robin(c, robin, len(knots))
         asm = sd.assemble_1d_bands if sd.enabled() else bs.assemble_1d_bands
         MK = [asm(p, T) for T in knots]
         Ms = [m for m, k in MK]
         Ks = [k for m, k in MK]
-        Ks[-1] = Ks[-1] + Ms[-1]
+        if robin is not None:
+            for a, (lo, hi) in enumerate(robin):
+                Ks[a] = Ks[a].copy()
+                Ks[a][0, p] += lo
+                Ks[a][-1, p] += hi
+        Ks[-1] = Ks[-1] + c * Ms[-1]
         A = cls(Ms, Ks)
         A.mass_bands = Ms
         return A
