@@ -273,6 +273,8 @@ int poms_dense_matvec(const double* Ainv, const double* x, double* y, int n, voi
  *  poms_assemble_1d: mass M and stiffness K bands (n, 2p+1) on the knot vector `knots` (n + p + 1
  *    entries) by Gauss-Legendre quadrature with the p+1 nodes / weights gauss_x, gauss_w on [-1, 1]
  *    (assembly_1d, sources/matrix_assembler.py:10-77; it computes K and returns only M, Appendix B).
+ *  poms_assemble_1d_advection: advection band G (n, 2p+1), G[i, k] = int B_{i+k-p}' B_i, with the same
+ *    knots and Gauss rule as poms_assemble_1d (the convection term beta_a G_a of -Lap u + beta.grad u + c u).
  *  poms_knot_insertion_rows: rows of the knot-insertion matrix P1 (n_f x n_c) between the nested knot
  *    vectors Tc, Tf by the Oslo recursion: P1[i, start[i] + w] = coef[i*(p+1) + w]
  *    (matrix_multi_stages, sources/mg_jac.py:67).
@@ -282,6 +284,8 @@ int poms_dense_matvec(const double* Ainv, const double* x, double* y, int n, voi
  */
 int poms_assemble_1d(const double* knots, int n, int p, const double* gauss_x, const double* gauss_w,
                      double* M, double* K, void* stream);
+int poms_assemble_1d_advection(const double* knots, int n, int p, const double* gauss_x, const double* gauss_w,
+                               double* G, void* stream);
 int poms_knot_insertion_rows(const double* Tc, int nc, const double* Tf, int nf, int p,
                              int32_t* start, double* coef, void* stream);
 int poms_band_lu_nopiv(const double* band, int n, int q, double* ab, int* info_dev, void* stream);

@@ -62,6 +62,7 @@ _PROTOS = {
                                         _i, _d, _vp, _vp, _vp]),
     "poms_color_add": (C.c_int, [_vp, _vp, _i, _i, _i, _l, _l, _i, _i, _vp]),
     "poms_assemble_1d": (C.c_int, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "poms_assemble_1d_advection": (C.c_int, [_vp, _i, _i, _vp, _vp, _vp, _vp]),
     "poms_knot_insertion_rows": (C.c_int, [_vp, _i, _vp, _i, _i, _vp, _vp, _vp]),
     "poms_band_lu_nopiv": (C.c_int, [_vp, _i, _i, _vp, _vp, _vp]),
     "poms_axis_dense_dmma": (C.c_int, [_vp, _vp, _vp, _i, _i, _l, _l, _l, _l, _l, _l, _vp]),

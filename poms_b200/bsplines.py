@@ -11,7 +11,7 @@ Band convention: (n, 2p+1) array, band[i, k] = A[i, i+k-p]
 """
 import numpy as np
 
-__all__ = ["make_open_knots", "assemble_1d_bands", "knot_insertion_rows", "rows_transpose",
+__all__ = ["make_open_knots", "assemble_1d_bands", "assemble_1d_advection", "knot_insertion_rows", "rows_transpose",
            "glt_band", "cardinal_bspline_values", "band_to_lapack", "band_lu", "pad_band",
            "band_to_dense", "dense_to_band"]
 
@@ -98,6 +98,30 @@ def assemble_1d_bands(p, T, toeplitz_interior=True):
         M[2 * p:n - 2 * p] = M[mid]
         K[2 * p:n - 2 * p] = K[mid]
     return M, K
+
+
+def assemble_1d_advection(p, T, toeplitz_interior=True):
+    """1-D advection band G (n, 2p+1), G[i, k] = int phi_{i+k-p}' phi_i, with the Gauss rule of
+    `assemble_1d_bands` (exact: the integrand has degree 2p-1).  G is not symmetric; integration by parts
+    gives G + G^T = e_{n-1} e_{n-1}^T - e_0 e_0^T on an open knot vector.  On uniform open knots rows
+    2p .. n-2p-1 are made bit-identical to the middle row, as in `assemble_1d_bands`."""
+    T = np.asarray(T, dtype=float)
+    n = len(T) - p - 1
+    spans = np.array([k for k in range(p, n) if T[k + 1] > T[k]], dtype=np.int64)
+    a, b = T[spans], T[spans + 1]
+    u, w = np.polynomial.legendre.leggauss(p + 1)
+    x = 0.5 * (a + b)[:, None] + 0.5 * (b - a)[:, None] * u[None, :]
+    wq = 0.5 * (b - a)[:, None] * w[None, :]
+    v, dv = _all_basis(T, p, spans, x)
+    Ge = np.einsum("eiq,ejq,eq->eij", v, dv, wq)          # Ge[e, il, jl] = int phi_jl' phi_il
+    G = np.zeros((n, 2 * p + 1))
+    for il in range(p + 1):
+        rows = spans - p + il
+        for jl in range(p + 1):
+            np.add.at(G, (rows, jl - il + p), Ge[:, il, jl])
+    if toeplitz_interior and n > 4 * p + 1 and _is_uniform_open(T, p):
+        G[2 * p:n - 2 * p] = G[n // 2]
+    return G
 
 
 def quadrature_tables(T, p):

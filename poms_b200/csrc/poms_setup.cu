@@ -1,6 +1,7 @@
 // poms_setup.cu -- device-side 1-D SETUP of the multigrid hierarchy (SURVEY.md section 8f-2):
 //   * poms_assemble_1d        1-D mass / stiffness bands by Gauss-Legendre quadrature
 //                             (/root/reference/sources/matrix_assembler.py:10-77, assembly_1d)
+//   * poms_assemble_1d_advection  1-D advection band G[i, k] = int B_{i+k-p}' B_i (convection term)
 //   * poms_knot_insertion_rows  rows of the knot-insertion (prolongation) matrix P1 by the Oslo
 //                             recursion (matrix_multi_stages, /root/reference/sources/mg_jac.py:67)
 //   * poms_band_lu_nopiv      banded LU without row interchanges in dgbtrf storage (the factor
@@ -39,16 +40,19 @@ __device__ __forceinline__ void basis_funs(const double* __restrict__ T, int p, 
     }
 }
 
-// one thread per band entry (i, k): M[i, i+k-p] = int B_i B_j, K = int B_i' B_j'
+// one thread per band entry (i, k), j = i+k-p: M[i, k] = int B_i B_j, K[i, k] = int B_i' B_j',
+// G[i, k] = int B_i B_j' (advection).  One quadrature loop serves both entry points; an output whose
+// pointer is null is neither computed into memory nor written.
 __global__ void __launch_bounds__(128) assemble_1d_kernel(const double* __restrict__ T, int n, int p,
                                                           const double* __restrict__ gx, const double* __restrict__ gw,
-                                                          double* __restrict__ M, double* __restrict__ K) {
+                                                          double* __restrict__ M, double* __restrict__ K,
+                                                          double* __restrict__ G) {
     const int W = 2 * p + 1;
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n * W) return;
     const int i = t / W, kk = t - i * W;
     const int j = i + kk - p;
-    double m = 0.0, s = 0.0;
+    double m = 0.0, s = 0.0, g = 0.0;
     if (j >= 0 && j < n) {
         const int e_lo = max(max(i, j), p), e_hi = min(min(i, j) + p, n - 1);
         for (int e = e_lo; e <= e_hi; ++e) {
@@ -69,23 +73,43 @@ __global__ void __launch_bounds__(128) assemble_1d_kernel(const double* __restri
                     if (r <= p - 1) d -= p * Nm[r] / (T[g + p + 1] - T[g + 1]);
                     return d;
                 };
+                const double djl = der(jl);
                 m = fma(w * N[il], N[jl], m);
-                s = fma(w * der(il), der(jl), s);
+                s = fma(w * der(il), djl, s);
+                g = fma(w * N[il], djl, g);
             }
         }
     }
-    M[t] = m;
-    K[t] = s;
+    if (M) M[t] = m;
+    if (K) K[t] = s;
+    if (G) G[t] = g;
+}
+
+static int launch_assemble_1d(const double* knots, int n, int p, const double* gauss_x, const double* gauss_w,
+                              double* M, double* K, double* G, void* stream) {
+    if (!knots || !gauss_x || !gauss_w) return bad_arg(1, "null pointer");
+    if (p < 1 || p > POMS_MAXP) return bad_arg(3, "p must be 1..5");
+    if (n < p + 1) return bad_arg(2, "n");
+    const int total = n * (2 * p + 1);
+    assemble_1d_kernel<<<(total + 127) / 128, 128, 0, (cudaStream_t)stream>>>(knots, n, p, gauss_x, gauss_w, M, K, G);
+    return 0;
 }
 
 extern "C" int poms_assemble_1d(const double* knots, int n, int p, const double* gauss_x, const double* gauss_w,
                                 double* M, double* K, void* stream) {
-    if (!knots || !gauss_x || !gauss_w || !M || !K) return bad_arg(1, "null pointer");
-    if (p < 1 || p > POMS_MAXP) return bad_arg(3, "p must be 1..5");
-    if (n < p + 1) return bad_arg(2, "n");
-    const int total = n * (2 * p + 1);
-    assemble_1d_kernel<<<(total + 127) / 128, 128, 0, (cudaStream_t)stream>>>(knots, n, p, gauss_x, gauss_w, M, K);
+    if (!M || !K) return bad_arg(1, "null pointer");
+    const int rc = launch_assemble_1d(knots, n, p, gauss_x, gauss_w, M, K, nullptr, stream);
+    if (rc) return rc;
     CHECK_LAUNCH("poms_assemble_1d");
+    return 0;
+}
+
+extern "C" int poms_assemble_1d_advection(const double* knots, int n, int p, const double* gauss_x,
+                                          const double* gauss_w, double* G, void* stream) {
+    if (!G) return bad_arg(1, "null pointer");
+    const int rc = launch_assemble_1d(knots, n, p, gauss_x, gauss_w, nullptr, nullptr, G, stream);
+    if (rc) return rc;
+    CHECK_LAUNCH("poms_assemble_1d_advection");
     return 0;
 }
 

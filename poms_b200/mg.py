@@ -11,9 +11,10 @@ Reference-faithful parts (SURVEY.md section 8a, a13-a17):
 
 EXTENSION beyond the reference (SURVEY.md section 8f-1; labelled in every report):
   * `Hierarchy`, `vcycle`, `mg_pcg`: recursive V-cycle used as the preconditioner of the
-    reference's own `pcg` driver.  Smoothers are the LINEAR, symmetric counterparts of the
-    reference's PCG smoothers -- a Chebyshev iteration preconditioned by damped-Jacobi's D^-1
-    ("jacobi") or by the GLT Kronecker solve T[m_{p-1}] (x) .. (x) T[m_{p-1}] ("glt",
+    reference's own `pcg` driver; `mg_gmres`: the same V-cycle preconditioning GMRES for the
+    non-symmetric convection-diffusion operator (`Hierarchy(beta=)`).  Smoothers are the LINEAR,
+    symmetric counterparts of the reference's PCG smoothers -- a Chebyshev iteration preconditioned
+    by damped-Jacobi's D^-1 ("jacobi") or by the GLT Kronecker solve T[m_{p-1}] (x) .. (x) T[m_{p-1}] ("glt",
     /root/reference/slides/content.tex:141-153) -- because a fixed SPD preconditioner is what CG
     needs (the reference's omega = 2/3 Jacobi diverges for p >= 3, see DESIGN.md).
 """
@@ -28,12 +29,12 @@ from . import bsplines as bs
 from . import profiling
 from .multilevels import knots_to_insert
 from .stencil import (StencilVectorSpace, StencilVector, KronSumMatrix, DeviceContext,
-                      _stream, EPI_STORE, EPI_RESID, EPI_DINV, EPI_AXPY, reaction_robin)
+                      _stream, EPI_STORE, EPI_RESID, EPI_DINV, EPI_AXPY, reaction_robin, convection_beta)
 from .kron_product import BandLU, kron_solve_bnd, kron_solve_bnd_update
 from . import solvers
 
 __all__ = ["Transfer", "DistTransfer", "CoarseSolver", "two_grid", "Hierarchy", "vcycle", "mg_pcg",
-           "fine_knots"]
+           "mg_gmres", "fine_knots"]
 
 
 def fine_knots(Tc, ts):
@@ -564,17 +565,21 @@ class Hierarchy:
 
     def __init__(self, p, N, ndim=None, Nc=8, device="cuda", smoother="glt", nu=1, ratio=4.0,
                  safety=1.1, slab=None, lengths=None, min_planes=32, coarsen="semi", setup="host",
-                 c=1.0, robin=None):
+                 c=1.0, robin=None, beta=None):
         """setup='device': the 1-D setup (assembly, knot-insertion rows, banded LU, eigenproblems)
         runs on the GPU (setup_device.py); 'host' (default): NumPy / SciPy.
         c, robin: reaction coefficient and Robin coefficients of every level's operator
-        (`KronSumMatrix.poisson`; ValueError for negative values or a singular operator)."""
+        (`KronSumMatrix.poisson`; ValueError for negative values or a singular operator).
+        beta: constant velocity (one component per axis) of a convection term beta . grad u.  Only the
+        fine-level operator `h.op` carries it; every level keeps the symmetric operator -Lap + c with
+        the same Robin faces, whose V-cycle preconditions `mg_gmres` (ValueError when the symmetric
+        part of `h.op` is not positive definite).  Without beta, `h.op` is `levels[0].A`."""
         if setup == "device":
             from . import setup_device as sd
             with sd.device_setup(True, device):
                 self.__init__(p, N, ndim=ndim, Nc=Nc, device=device, smoother=smoother, nu=nu, ratio=ratio,
                               safety=safety, slab=slab, lengths=lengths, min_planes=min_planes,
-                              coarsen=coarsen, setup="host", c=c, robin=robin)
+                              coarsen=coarsen, setup="host", c=c, robin=robin, beta=beta)
             self.setup = "device"
             return
         self.setup = "host"
@@ -585,6 +590,11 @@ class Hierarchy:
         self.lengths = [1.0] * len(N) if lengths is None else [float(v) for v in lengths]
         self.p, self.ndim = p, len(N)
         self.c, self.robin = reaction_robin(c, robin, self.ndim)
+        self.beta = convection_beta(beta, self.ndim)
+        if self.beta is not None:
+            # built (and checked) first, so that a rejected velocity costs no hierarchy
+            fine_knots_ = [bs.make_open_knots(p, n + p) * L for n, L in zip(N, self.lengths)]
+            op = KronSumMatrix.poisson(p, fine_knots_, c=self.c, robin=self.robin, beta=self.beta)
         self.device = torch.device(device)
         self.smoother, self.nu, self.ratio, self.safety = smoother, nu, ratio, safety
         self.levels = []
@@ -627,6 +637,7 @@ class Hierarchy:
                 f.transfer = DistTransfer(c.knots, f.knots, p, self.device, slab, c.distributed)
             else:
                 f.transfer = Transfer(c.knots, f.knots, p, self.device)
+        self.op = self.levels[0].A if self.beta is None else op
         self.coarse = CoarseSolver(self.levels[-1].A, self.device)
         for lv in self.levels[:-1]:
             self._setup_smoother(lv)
@@ -969,6 +980,9 @@ def mg_pcg(h, b, x0=None, tol=1e-10, maxiter=200, criterion="relative", verbose=
     On one device the iteration runs as two CUDA graphs (`_PcgGraphs`; POMS_B200_GRAPH=0 or an
     enabled profiler selects the launch-by-launch driver); the returned x is then the hierarchy's
     persistent solution vector, overwritten by the next solve on the same hierarchy."""
+    if h.beta is not None:
+        raise ValueError("mg_pcg needs a symmetric operator: a hierarchy with a convection term (beta) is "
+                         "solved by mg_gmres")
     A = h.levels[0].A
 
     def psolve(A_, r):
@@ -1004,3 +1018,19 @@ def mg_pcg(h, b, x0=None, tol=1e-10, maxiter=200, criterion="relative", verbose=
     info["success"] = bool(info["res_norm"] ** 2 <= target)
     info["graphed"] = bool(graphed)
     return x, info
+
+
+def mg_gmres(h, b, x0=None, tol=1e-10, maxiter=300, restart=30):
+    """Solve h.op x = b (the convection-diffusion operator of `Hierarchy(beta=)`, or the symmetric one)
+    by `solvers.gmres` with right preconditioning by one V-cycle of the symmetric hierarchy.  The V-cycle
+    from a zero guess is a fixed linear map (what GMRES needs of its preconditioner), spectrally
+    equivalent to h.op at fixed beta and c, so the iteration count does not grow with the grid.  Its
+    result lives in the hierarchy's workspace, which the next cycle overwrites, so it is copied into a
+    vector that gmres owns.  Works on slab-partitioned hierarchies (the dots of gmres are all-reduced,
+    the mat-vecs exchange halos).  Returns (x, info) like mg_pcg:
+    info['res_norm'] is the true residual ||b - h.op x|| (gmres recomputes it before it stops), and
+    info['success'] says whether it is <= tol * ||b - h.op x0||."""
+    def psolve(A_, v):
+        return vcycle(h, 0, v).copy()
+
+    return solvers.gmres(h.op, b, x0=x0, tol=tol, maxiter=maxiter, restart=restart, psolve=psolve)

@@ -4,6 +4,7 @@
 implementations (bsplines.py, the default: they are what the golden-vector parity tests pin) to
 hand-written CUDA kernels for the O(n p^2) parts
     assembly of the 1-D mass / stiffness bands   /root/reference/sources/matrix_assembler.py:10-77
+    (and of the advection band of the convection term)
     knot-insertion rows of P1 (Oslo recursion)   /root/reference/sources/mg_jac.py:67
     banded LU of the GLT matrices (no pivoting)  /root/reference/sources/kron_product.py:191-197
 and to torch.linalg on the device (cuSOLVER: library calls, setup only) for the dense generalised
@@ -58,6 +59,22 @@ def assemble_1d_bands(p, T, toeplitz_interior=True):
         M[2 * p:n - 2 * p] = M[mid].clone()
         K[2 * p:n - 2 * p] = K[mid].clone()
     return M.cpu().numpy(), K.cpu().numpy()
+
+
+def assemble_1d_advection(p, T, toeplitz_interior=True):
+    """Device twin of bsplines.assemble_1d_advection: returns the host band G (n, 2p+1)."""
+    T = np.asarray(T, dtype=np.float64)
+    n = len(T) - p - 1
+    dev = _device
+    Td = torch.as_tensor(T, device=dev)
+    u, w = np.polynomial.legendre.leggauss(p + 1)
+    ud, wd = torch.as_tensor(u, device=dev), torch.as_tensor(w, device=dev)
+    G = torch.empty((n, 2 * p + 1), dtype=torch.float64, device=dev)
+    _lib.check(_lib.lib().poms_assemble_1d_advection(Td.data_ptr(), n, p, ud.data_ptr(), wd.data_ptr(),
+                                                      G.data_ptr(), _stream()), "poms_assemble_1d_advection")
+    if toeplitz_interior and n > 4 * p + 1 and bs._is_uniform_open(T, p):
+        G[2 * p:n - 2 * p] = G[n // 2].clone()
+    return G.cpu().numpy()
 
 
 def knot_insertion_rows(Tc, Tf, p):

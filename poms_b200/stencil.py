@@ -629,6 +629,64 @@ def reaction_robin(c, robin, ndim):
     return c, robin
 
 
+def convection_beta(beta, ndim):
+    """Checked velocity of `KronSumMatrix.poisson`: None, or a list of ndim finite floats (ValueError)."""
+    if beta is None:
+        return None
+    try:
+        vals = [float(v) for v in beta]
+    except (TypeError, ValueError):
+        raise ValueError("beta must be None or %d numbers (one velocity component per axis)" % ndim) from None
+    if len(vals) != ndim:
+        raise ValueError("beta must have one component per axis (%d), got %d" % (ndim, len(vals)))
+    if not all(np.isfinite(v) for v in vals):
+        raise ValueError("beta must be finite (got %r)" % (vals,))
+    return vals
+
+
+def _gen_eig_min(Sb, Mb, lower):
+    """Smallest generalised eigenvalue of S x = l M x for a symmetric band S (possibly indefinite) and the
+    SPD mass band M (host), given a lower bound `lower` of it.  n <= 1500: dense LAPACK; above: shift-invert
+    Lanczos (sparse LU of S - s M) at a shift s below `lower`, the same size split as `mg._gen_eig_max`."""
+    n = Sb.shape[0]
+    if n <= 1500:
+        from scipy.linalg import eigh
+        return float(eigh(bs.band_to_dense(Sb), bs.band_to_dense(Mb), eigvals_only=True,
+                          subset_by_index=[0, 0])[0])
+    import scipy.sparse as sp
+    from scipy.sparse.linalg import eigsh
+
+    def csc(band):
+        p = (band.shape[1] - 1) // 2
+        diags = [band[max(0, -k):n - max(0, k), k + p] for k in range(-p, p + 1)]
+        return sp.diags(diags, list(range(-p, p + 1)), shape=(n, n), format="csc")
+    v0 = np.cos(np.arange(n) * 0.7) + 1.5          # deterministic start vector
+    return float(eigsh(csc(Sb), k=1, M=csc(Mb), sigma=lower - 1.0, which="LM", v0=v0,
+                       return_eigenvectors=False)[0])
+
+
+def symmetric_part_lmin(Ks, Ms, c, beta, lengths):
+    """lambda_min(A_s, M (x) .. (x) M) of the operator with the bands Ks (K_a + R_a, without c M and
+    without the advection), Ms and the axis lengths L_a: A_s = sum_a S_a (x) M_others + c M (x) .. (x) M
+    with S_a = K_a + R_a + (beta_a / 2)(E_hi - E_lo), because G_a + G_a^T = E_hi - E_lo.  All factors are
+    symmetric and share M, so the value is c + sum_a lambda_min(S_a, M_a): d 1-D problems.
+
+    Lower bound of a 1-D value (the shift of the sparse path): Galerkin eigenvalues are bounded below by
+    the continuous ones, and u(x0)^2 <= e |u'|^2 + (1/e + 1/L) |u|^2 with e = 2 / |beta| gives
+    lambda_min(S_a, M_a) >= -(beta^2 / 4 + |beta| / (2 L))."""
+    lam = c
+    for a, (K, M) in enumerate(zip(Ks, Ms)):
+        S = np.array(K, dtype=np.float64)
+        b = beta[a] if beta is not None else 0.0
+        p = (S.shape[1] - 1) // 2
+        S[0, p] -= 0.5 * b
+        S[-1, p] += 0.5 * b
+        la = _gen_eig_min(S, M, -(0.25 * b * b + 0.5 * abs(b) / lengths[a]))
+        # K_a + R_a is positive semi-definite: a rounding-level negative value of a pure Neumann axis is 0
+        lam += max(la, 0.0) if b == 0.0 else la
+    return lam
+
+
 class KronSumMatrix:
     """Kronecker-structured operator on a d-dim tensor-product space (d = 2, 3).
 
@@ -663,20 +721,27 @@ class KronSumMatrix:
         self._dev = {}
 
     @classmethod
-    def poisson(cls, p, knots, c=1.0, robin=None):
-        """-Lap(u) + c u with du/dn + alpha u = 0 on the boundary (the weak form's natural condition)
-        on the tensor-product space with the given per-axis knot vectors.  The defaults (c = 1, no
-        Robin term) are the operator `assembly_2d` builds (/root/reference/sources/matrix_assembler.py:
-        82-179), K(x)M + M(x)(K+M) [2-D] / K(x)M(x)M + M(x)K(x)M + M(x)M(x)(K+M) [3-D].
+    def poisson(cls, p, knots, c=1.0, robin=None, beta=None):
+        """-Lap(u) + beta . grad(u) + c u with du/dn + alpha u = 0 on the boundary (the weak form's natural
+        condition) on the tensor-product space with the given per-axis knot vectors.  The defaults (c = 1,
+        no Robin term, no convection) are the operator `assembly_2d` builds (/root/reference/sources/
+        matrix_assembler.py:82-179), K(x)M + M(x)(K+M) [2-D] / K(x)M(x)M + M(x)K(x)M + M(x)M(x)(K+M) [3-D].
 
         robin: None, or one pair (alpha_lo, alpha_hi) per axis: alpha int_F u v ds on the faces
         x_a = T_a[p] and x_a = T_a[n_a].  On an open knot vector only the first (last) basis function
         is non-zero there, with value 1, so the face term is (alpha e e^T) (x) M_others: one diagonal
         entry of K_a.  c M(x)..(x)M goes into the last K as K + c M.  Both keep the Kronecker-sum
         form and change no interior row.  c >= 0, alpha >= 0, and c > 0 or some alpha > 0 (otherwise
-        the operator is singular): ValueError."""
+        the operator is singular): ValueError.
+
+        beta: None, or one constant velocity component per axis: int (beta . grad u) v = sum_a beta_a
+        G_a (x) M_others with the 1-D advection band G_a (`bsplines.assemble_1d_advection`), added into
+        K_a.  The operator is then not symmetric; its symmetric part must be positive definite (checked
+        from d 1-D eigenproblems, `symmetric_part_lmin`), otherwise ValueError: an inflow face
+        (beta . n < 0) needs enough of alpha or c."""
         from . import setup_device as sd
         c, robin = reaction_robin(c, robin, len(knots))
+        beta = convection_beta(beta, len(knots))
         asm = sd.assemble_1d_bands if sd.enabled() else bs.assemble_1d_bands
         MK = [asm(p, T) for T in knots]
         Ms = [m for m, k in MK]
@@ -686,6 +751,18 @@ class KronSumMatrix:
                 Ks[a] = Ks[a].copy()
                 Ks[a][0, p] += lo
                 Ks[a][-1, p] += hi
+        if beta is not None:
+            lengths = [float(T[-1] - T[0]) for T in knots]
+            lam = symmetric_part_lmin(Ks, Ms, c, beta, lengths)
+            if not lam > 0.0:
+                raise ValueError(
+                    "the symmetric part of -Lap u + beta.grad u + c u with these Robin terms is not positive "
+                    "definite (lambda_min = %.3e): an inflow face (beta . n < 0) needs alpha + c large enough "
+                    "(e.g. alpha >= |beta_a| / 2 there)" % lam)
+            adv = sd.assemble_1d_advection if sd.enabled() else bs.assemble_1d_advection
+            for a, b in enumerate(beta):
+                if b != 0.0:
+                    Ks[a] = Ks[a] + b * adv(p, knots[a])
         Ks[-1] = Ks[-1] + c * Ms[-1]
         A = cls(Ms, Ks)
         A.mass_bands = Ms
